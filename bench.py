@@ -11,6 +11,10 @@ synthetic scene (~2.87 M triangles, 1 106 instances, 20 050 emissive triangles),
   python bench.py --impl reference --steps K --warmup W    # the reference algorithm on the host CPU
                                                            # (oracle port; oracle/_ref is unbuildable)
 
+--steps K sets the frames of every timed loop.  --dump-outputs DIR writes what the timed path computed in its last step, the
+1920x1080 RGBA float32 beauty framebuffer, to DIR/beauty.npy; the scene, the camera and the per-frame seeds are fixed, so two
+builds run with the same arguments can be compared output for output.
+
 One JSON line on stdout (rank 0).  `value` = rays traced by the whole job per second with
 everything resident in HBM; `e2e` = the same through the C ABI with per-frame host->device uploads
 (instance table + parameter blocks from pinned memory) and the device->host read of the beauty
@@ -309,7 +313,7 @@ def measure_nrc_and_svgf(ctx, scene, args):
         pc.numAccumFrames = f
         driver.render_restir_nrc_frame(f, [int(rng.integers(0, 2 ** 32)) for _ in range(2)])
 
-    n_warm, n_frames = 16, max(args.steps, 8)
+    n_warm, n_frames = 16, args.steps
     for f in range(n_warm):
         combined_frame(f)
     torch.cuda.synchronize()
@@ -355,7 +359,7 @@ def measure_nrc_and_svgf(ctx, scene, args):
     # ---- SVGF (config 4) on the ReSTIR DI output
     ren = engine.ReSTIRRenderer(ctx, scene, WIDTH, HEIGHT)
     svgf_ms = []
-    for f in range(10):
+    for f in range(3 + args.steps):  # the first three frames warm up
         ren.render_frame()
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
@@ -410,7 +414,7 @@ def measure_config5(scene, args, rank, world, local_rank):
     torch.cuda.synchronize()
     driver.check_peers()
     ctx.read_stats(reset=True)
-    n_frames = max(args.steps, 8)
+    n_frames = args.steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(n_frames):
@@ -543,6 +547,12 @@ def run_gpu(args):
     clocks = sampler.stop()
     ms_total = ev0.elapsed_time(ev1)
     rays = ctx.read_stats(reset=True)[0]
+    # --dump-outputs: what the timed path computed in its last step, the beauty framebuffer a caller of the frame receives
+    # (at N > 1 the composited frame every rank holds after the all-gather)
+    last_beauty = None
+    if args.dump_outputs and rank == 0:
+        last_beauty = (driver.composited.cpu().numpy().reshape(HEIGHT, WIDTH, 4) if driver is not None
+                       else ctx.download(abi.BUF_BEAUTY_ACCUM))
     # the G-buffer halo rows a rank recomputes for the spatial pass are redundant work, not throughput: their primary rays
     # are not counted (so `value` at N > 1 is the same frame's rays as at N = 1, over a shorter time)
     halo_rays_per_frame = 0
@@ -762,6 +772,9 @@ def run_gpu(args):
         line["config5"] = config5
     if cpu_baseline is not None:
         line["cpu_baseline"] = cpu_baseline
+    if last_beauty is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "beauty.npy"), np.ascontiguousarray(last_beauty, dtype=np.float32))
     emit_line(line)
     if world > 1:
         dist.destroy_process_group()
@@ -799,7 +812,13 @@ def main():
     ap.add_argument("--rays-per-px", type=float, default=2.883, help="--impl reference: rays per pixel (GPU-counted)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the NRC / north-star / SVGF measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the beauty framebuffer of the last timed frame to DIR/beauty.npy (float32 [H, W, 4])")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "gfxb200":
+        ap.error("--dump-outputs writes the CUDA path's frame: --impl gfxb200 only")
     if args.impl == "reference":
         run_reference(args)
     else:

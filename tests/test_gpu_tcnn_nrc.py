@@ -1,7 +1,9 @@
 """The NRC network against the reference's own code on the GPU: tiny-cuda-nn's NetworkWithInputEncoding + Trainer built from
 neural_radiance_caching/network_interface.cu's config (oracle/ref_tcnn/tcnn_nrc.cu -> oracle/_ref/libtcnn_nrc.so, compiled from
-/root/reference/ext/tiny-cuda-nn where it lies).  tests/tcnn_nrc_check.py does the work in a child process (third-party kernels)
-and prints one JSON line; the bars:
+the reference's vendored tiny-cuda-nn).  Its outputs on the check's seeded inputs are stored in tests/golden/golden_tcnn_nrc.npz
+(written by `python tests/tcnn_nrc_check.py --write-golden`; a fixed sample of the rows and parameters, the initial parameters as
+digests), so the test needs no reference build.  tests/tcnn_nrc_check.py does the work in a child process and prints one JSON
+line; the relative L2 bars against tiny-cuda-nn hold over the stored sample:
 
   * gfx_nrc_create's initial parameters == tcnn::Trainer{seed 1337}'s, every fp32 master weight bit for bit;
   * inferred radiance within 1e-3 relative L2 of tiny-cuda-nn's (BASELINE.json north_star), before and after four training steps;
@@ -22,18 +24,17 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, "tests", "golden", "golden_tcnn_nrc.npz")
 
 
 def test_nrc_network_matches_tiny_cuda_nn():
-    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libtcnn_nrc.so")):
-        pytest.skip("oracle/_ref/libtcnn_nrc.so not built (needs /root/reference at build time)")
-    proc = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "tcnn_nrc_check.py"), "--no-timing"], capture_output=True,
+    proc = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "tcnn_nrc_check.py"), "--golden", GOLDEN], capture_output=True,
                           text=True, timeout=400)
     line = proc.stdout.strip().splitlines()[-1] if proc.stdout.strip() else ""
     assert proc.returncode == 0, f"rc={proc.returncode} {line[:400]} {proc.stderr[-600:]}"
     r = json.loads(line)
     init = r["init"]
-    assert init["master_mismatches"] == 0 and init["training_half_mismatches"] == 0 and init["inference_all_zero"], init
+    assert init["master_equal"] and init["training_half_equal"] and init["inference_all_zero"], init
     fwd = r["forward"]
     assert fwd["ours_vs_tcnn"] <= 1e-3, fwd
     assert fwd["oracle_halfacc_vs_tcnn"] <= 1e-4, fwd

@@ -4,6 +4,8 @@
  * bvh::traverse (first-found and canonical tie-break) equals the exhaustive brute-force closest hit,
  * any-hit equals "brute-force closest hit exists in range".
 """
+import os
+
 import numpy as np
 import pytest
 
@@ -79,12 +81,17 @@ def test_node_codec_is_conservative(tiny):
     assert (nodes["childQMin"][:, :, :].transpose(0, 2, 1)[valid] <= nodes["childQMax"].transpose(0, 2, 1)[valid]).all()
 
 
-def test_teapot_config1_build(oracle):
-    import os
-    path = "/root/reference/data/teapot.obj"
-    scene = scenes.teapot_like_scene(path if os.path.exists(path) else None)
+def test_teapot_config1_build(oracle, tmp_path):
+    """config 1's teapot (tests/golden/teapot.npz, written by make_teapot.py), written back as an OBJ so that it goes through
+    scenes.load_obj like the original file"""
+    teapot = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "teapot.npz"))
+    faces = np.cumsum(teapot["face_deltas"].astype(np.int64)).reshape(-1, 3) + 1
+    path = tmp_path / "teapot.obj"
+    with open(path, "w") as fh:
+        fh.writelines("v %.9g %.9g %.9g\n" % tuple(float(x) for x in v) for v in teapot["positions"])
+        fh.writelines("f %d %d %d\n" % tuple(f) for f in faces)
+    scene = scenes.teapot_like_scene(str(path))
     oscene = oracle.OracleScene(scene)
     info = oscene.info()
-    if os.path.exists(path):
-        assert info.numTriangles == 15704 + 2  # SURVEY.md §0: 15 704 faces + the rectangle light
+    assert info.numTriangles == 15704 + 2  # SURVEY.md §0: 15 704 faces + the rectangle light
     assert oscene.validate() == ""
