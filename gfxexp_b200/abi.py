@@ -422,7 +422,7 @@ EXPORTED_SYMBOLS = tuple(_DECLS.keys())
 def load_library(path: str | None = None) -> C.CDLL:
     """Load libgfxb200.so and attach prototypes.  Raises OSError if the CUDA extension has not been
     built (python -c 'import __graft_entry__ as g; g.build()') — there is no fallback path."""
-    path = path or os.environ.get("GFXB200_LIB") or LIB_PATH  # GFXB200_LIB: A/B builds of the same library
+    path = path or os.environ.get("GFXB200_LIB") or LIB_PATH  # GFXB200_LIB: another build of the library, e.g. to compare two commits
     if not os.path.exists(path):
         raise OSError(f"{path} not found: build the CUDA extension first (__graft_entry__.build()); "
                       "gfxexp_b200 has no CPU fallback")

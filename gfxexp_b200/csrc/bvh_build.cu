@@ -21,9 +21,6 @@
 #include "scene.cuh"
 #include "context.h"
 #include <cub/cub.cuh>
-#include <chrono>
-#include <cstdio>
-#include <cstdlib>
 
 namespace gfx {
 
@@ -1232,9 +1229,7 @@ int buildBvh(gfx_ctx* ctx, cudaStream_t stream, uint32_t flags) {
         ha.blockRight = hugeBlockStore + hugeMaxBlocks;
         int cur = 0;
         uint32_t depth = 0;
-        const bool profile = getenv("GFX_BVH_SAH_PROFILE") != nullptr;
         while (sizes[0] + sizes[1] + sizes[2] > 0) {
-            const auto t0 = std::chrono::steady_clock::now();
             sa.smallOut = smallLists[cur ^ 1];
             sa.bigOut = bigLists[cur ^ 1];
             sa.hugeOut = hugeLists[cur ^ 1];
@@ -1265,9 +1260,6 @@ int buildBvh(gfx_ctx* ctx, cudaStream_t stream, uint32_t flags) {
             }
             GFX_CUDA(ctx, cudaMemcpyAsync(hostSah, counters, 16, cudaMemcpyDeviceToHost, stream));
             GFX_CUDA(ctx, cudaStreamSynchronize(stream));
-            if (profile)
-                fprintf(stderr, "sah level %u: %u small + %u big + %u huge nodes, %.3f ms\n", depth, sizes[0], sizes[1], sizes[2],
-                        std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
             sizes[0] = hostSah[0];
             sizes[1] = hostSah[1];
             sizes[2] = hostSah[3];

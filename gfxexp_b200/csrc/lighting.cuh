@@ -140,24 +140,6 @@ GFX_D F8 pickGuideFetch(const DevScene &s, float ul) { // the guide entry of ul'
     const uint32_t b = min(dm_f2uint(ul * (float)kPickGuideSize), kPickGuideSize - 1); // exact: a power-of-two product, floored
     return ldg256(s.pickGuide + 2 * (size_t)b);
 }
-GFX_D LightPick pickLightFromGuide(const DevScene &s, float ul, const F8 &g);
-GFX_D LightPick pickLight(const DevScene &s, float ul) {
-#ifndef GFX_AB_CHAIN_PICK
-    return pickLightFromGuide(s, ul, pickGuideFetch(s, ul));
-#else
-    LightPick r;
-    // A/B (-DGFX_AB_CHAIN_PICK): the definition instead of its flattened form
-    float unusedProb;
-    r.key = chainPickLightTriangle(s, ul, &unusedProb);
-    if (!(r.key & kPickNone)) {
-        const F8 h0 = ldg256(s.lightTris + kLightTriStride * (size_t)r.key);
-        r.sphere = h0.lo;
-        r.density = h0.hi.x;
-        r.instSlot = __float_as_uint(h0.hi.y);
-    }
-    return r;
-#endif
-}
 GFX_D LightPick pickLightFromGuide(const DevScene &s, float ul, const F8 &g) {
     LightPick r;
     const uint32_t head = __float_as_uint(g.lo.x);
@@ -190,6 +172,7 @@ GFX_D LightPick pickLightFromGuide(const DevScene &s, float ul, const F8 &g) {
     }
     return r;
 }
+GFX_D LightPick pickLight(const DevScene &s, float ul) { return pickLightFromGuide(s, ul, pickGuideFetch(s, ul)); }
 GFX_D uint32_t pickLightTriangle(const DevScene &s, float ul) { return pickLight(s, ul).key; }
 
 // A Low-Distortion Map Between Triangle and Square (restir_di_shared.h:485-498)
@@ -400,12 +383,7 @@ GFX_D bool sampleLightUnlessDark(const DevScene &s, float ul, float u0, float u1
         const float r = pick.sphere.w;
         const float t = -(dot(dc, shadingNormal) * vOutLocalZ);          // > 0: centre on the far side of the surface
         const float margin = t - 1.001f * r * fabsf(vOutLocalZ);
-#ifdef GFX_AB_NO_SPHERE
-        const bool sphereCull = false;
-#else
-        const bool sphereCull = true;
-#endif
-        if (sphereCull && r >= 0.0f && margin > 0.0f && margin * margin > 8e-6f * (sqLength(dc) + r * r) * (vOutLocalZ * vOutLocalZ)) {
+        if (r >= 0.0f && margin > 0.0f && margin * margin > 8e-6f * (sqLength(dc) + r * r) * (vOutLocalZ * vOutLocalZ)) {
             *areaPDensity = 1.0f; // any positive number: the caller only asks whether the density is positive
             return true;
         }

@@ -324,24 +324,15 @@ __global__ void __launch_bounds__(128) k_nrcInfer(NrcLevels levels, const __half
     const uint32_t warp = tid >> 5;
     const uint32_t weightBytes = (numHiddenLayers * kWidth * kWidth + kPaddedOutput * kWidth) * 2;
 
-    // resident weights (18 KB, once per persistent CTA): cooperative 16-byte copies. -DGFX_NRC_INFER_TMA switches to one
-    // cp.async.bulk + mbarrier like the training kernel; measured neutral for the copy itself and 7 % slower overall
-    // because of the code ptxas then generates for the encoder (profiles/r01_summary.md), so it is off here.
-    __shared__ __align__(8) uint64_t weightBar;
+    // resident weights (18 KB, once per persistent CTA): cooperative 16-byte copies.  One cp.async.bulk + mbarrier like the
+    // training kernel measured neutral for the copy itself and 7 % slower overall because of the code ptxas then generates
+    // for the encoder (profiles/r01_summary.md).
     if (tid == 0) {
         mbarInit(&bar, 1);
-        mbarInit(&weightBar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-#ifdef GFX_NRC_INFER_TMA
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smemU32(&weightBar)), "r"(weightBytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     :: "r"(smemU32(sW)), "l"(ummaWeights), "r"(weightBytes), "r"(smemU32(&weightBar)) : "memory");
-#endif
     }
-#ifndef GFX_NRC_INFER_TMA
     for (uint32_t i = tid; i < weightBytes / 16; i += 128)
         reinterpret_cast<uint4*>(sW)[i] = __ldg(ummaWeights + i);
-#endif
     if (warp == 0) { // TMEM: 64 fp32 accumulator columns x 128 lanes
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smemU32(&tmemBaseShared)), "r"(64u) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
@@ -350,9 +341,6 @@ __global__ void __launch_bounds__(128) k_nrcInfer(NrcLevels levels, const __half
     tcFenceBefore();
     __syncthreads();
     tcFenceAfter();
-#ifdef GFX_NRC_INFER_TMA
-    mbarWait(&weightBar, 0); // the weight blob has landed (async proxy write: visible to tcgen05.mma without a proxy fence)
-#endif
     const uint32_t tmemBase = tmemBaseShared;
     const uint32_t tmemRow = tmemBase + ((warp * 32u) << 16); // this warp's 32 lanes
 
@@ -1598,11 +1586,10 @@ static int nrcInferLaunch(gfx_nrc* n, cudaStream_t s, const float* inputData, fl
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const uint32_t numTiles = numData / kTileRows; // upper bound when numDataPtr is given
-    // GFX_NRC_INFER_FUSED=1: the one-kernel form (encode by L2 gathers inside the MLP kernel), the A/B arm; it is also the
-    // path for buffers the TMA bulk copies cannot take (not 16-byte aligned)
-    const char* fusedEnv = getenv("GFX_NRC_INFER_FUSED");
+    // buffers the TMA bulk copies cannot take (not 16-byte aligned) go through the one-kernel form: encode by L2 gathers
+    // inside the MLP kernel
     const bool aligned = (reinterpret_cast<uintptr_t>(inputData) & 15u) == 0 && (reinterpret_cast<uintptr_t>(predictionData) & 15u) == 0;
-    if ((fusedEnv && fusedEnv[0] == '1') || !aligned) {
+    if (!aligned) {
         const size_t smem = kATileBytes + (size_t)n->numMatrixWeights * 2;
         NRC_CUDA(n, cudaFuncSetAttribute(k_nrcInfer, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         const uint32_t grid = numTiles < (uint32_t)sms * 6 ? numTiles : (uint32_t)sms * 6;
@@ -1738,10 +1725,8 @@ int gfx_nrc_train(gfx_nrc* n, void* stream, const float* inputData, const float*
     cudaStream_t s = (cudaStream_t)stream;
     NRC_CUDA(n, cudaMemsetAsync(n->loss, 0, 4, s));
     // Fully-connected layers on tcgen05 (forward, data gradient and weight gradient); the CUDA-core kernel stays for deep
-    // networks whose activation tiles do not fit in shared memory and as the A/B switch GFX_NRC_TRAIN_CUDACORES=1.
-    const char* cudaCoresEnv = getenv("GFX_NRC_TRAIN_CUDACORES");
-    const bool forceCudaCores = cudaCoresEnv && cudaCoresEnv[0] == '1';
-    if (n->numHiddenLayers <= 3 && !forceCudaCores) {
+    // networks (more than 3 hidden layers) whose activation tiles do not fit in shared memory.
+    if (n->numHiddenLayers <= 3) {
         const size_t smem = (size_t)n->numMatrixWeights * 4 + (size_t)(n->numHiddenLayers + 1) * kATileBytes + 3 * (size_t)kATileBytes;
         NRC_CUDA(n, cudaFuncSetAttribute(k_nrcTrainTc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         { GFX_TIMED(n->ctx, s, "nrc_train_prep_weights");

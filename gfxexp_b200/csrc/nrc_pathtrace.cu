@@ -16,13 +16,6 @@
 // neural_radiance_caching_main.cpp:2291-2304; here the inference launch reads its size from device memory).
 #include "pathtrace.cuh"
 
-// occupancy of the first-hit / bounce kernels: 16 blocks of 64 threads per SM = 64 registers (measured against the 88-128
-// ptxas picks unconstrained: path-tracer bounce 0.44 -> 0.37 ms, NRC bounce 0.58 -> 0.53 ms; profiles/r02_summary.md)
-#ifndef GFX_BOUNCE_MIN_BLOCKS
-#define GFX_BOUNCE_MIN_BLOCKS 16
-#endif
-#define GFX_BOUNCE_BOUNDS __launch_bounds__(64, GFX_BOUNCE_MIN_BLOCKS)
-
 namespace gfx {
 
 constexpr float kPathTerminationFactor = 0.01f;        // neural_radiance_caching_shared.h:7
@@ -285,7 +278,7 @@ GFX_D void emitRaysNrc(const DevScene &s, const DevPathState &ps, const DevNrc &
 }
 
 // pathTrace_raygen_generic<true> up to the path extension loop (optix_pathtracing_kernels.cu:95-283)
-__global__ void GFX_BOUNCE_BOUNDS k_nrcFirstHit(DevScene s, DevFrame f, DevFrameParams p, DevPathState ps, DevNrc n) {
+__global__ void __launch_bounds__(64, kBounceMinBlocks) k_nrcFirstHit(DevScene s, DevFrame f, DevFrameParams p, DevPathState ps, DevNrc n) {
     const uint32_t x = blockIdx.x * 8 + threadIdx.x;
     const uint32_t y = p.y0 + blockIdx.y * 8 + threadIdx.y;
     const uint32_t lane = (threadIdx.x + threadIdx.y * blockDim.x) & 31u;
@@ -364,7 +357,7 @@ __global__ void GFX_BOUNCE_BOUNDS k_nrcFirstHit(DevScene s, DevFrame f, DevFrame
 }
 
 // pathTrace_closestHit_generic<true> (:363-623) + the loop bookkeeping (:285-311) on the queue of live paths
-__global__ void GFX_BOUNCE_BOUNDS k_nrcBounce(DevScene s, DevFrame f, DevFrameParams p, DevPathState ps, DevNrc n, uint32_t round) {
+__global__ void __launch_bounds__(64, kBounceMinBlocks) k_nrcBounce(DevScene s, DevFrame f, DevFrameParams p, DevPathState ps, DevNrc n, uint32_t round) {
     const uint32_t curQueue = round & 1u, nextQueue = curQueue ^ 1u;
     const uint32_t* roundCounters = ps.counters + 4 * round;
     uint32_t* nextCounters = ps.counters + 4 * (round + 1);

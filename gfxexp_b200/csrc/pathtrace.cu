@@ -22,13 +22,6 @@
 // float4 planes indexed by pixel.  The RNG draw order of every pixel is the reference's.
 #include "pathtrace.cuh"
 
-// occupancy of the first-hit / bounce kernels: 16 blocks of 64 threads per SM = 64 registers (measured against the 88-128
-// ptxas picks unconstrained: path-tracer bounce 0.44 -> 0.37 ms, NRC bounce 0.58 -> 0.53 ms; profiles/r02_summary.md)
-#ifndef GFX_BOUNCE_MIN_BLOCKS
-#define GFX_BOUNCE_MIN_BLOCKS 16
-#endif
-#define GFX_BOUNCE_BOUNDS __launch_bounds__(64, GFX_BOUNCE_MIN_BLOCKS)
-
 namespace gfx {
 
 // One path vertex: NEE + next direction.  The ReGIR variant (regir/gpu_kernels/optix_pathtracing_kernels.cu) draws its
@@ -62,7 +55,7 @@ GFX_D void shadeVertexVariant(const DevScene &s, const DevRegir &rg, const DevFr
 
 // pathTrace_rayGen_generic up to the path extension loop (:73-160)
 template <bool REGIR>
-__global__ void GFX_BOUNCE_BOUNDS k_ptFirstHit(DevScene s, DevFrame f, DevFrameParams p, DevPathState ps, DevRegir rg) {
+__global__ void __launch_bounds__(64, kBounceMinBlocks) k_ptFirstHit(DevScene s, DevFrame f, DevFrameParams p, DevPathState ps, DevRegir rg) {
     const uint32_t x = blockIdx.x * 8 + threadIdx.x;
     const uint32_t y = p.y0 + blockIdx.y * 8 + threadIdx.y;
     const uint32_t lane = (threadIdx.x + threadIdx.y * blockDim.x) & 31u;
@@ -113,7 +106,7 @@ __global__ void GFX_BOUNCE_BOUNDS k_ptFirstHit(DevScene s, DevFrame f, DevFrameP
 // pathTrace_closestHit_generic (:218-300) + the bookkeeping of the path extension loop (:161-194) for the
 // compacted queue of live paths; `round` = pathLength - 2 selects the queue parity and the counters.
 template <bool REGIR>
-__global__ void GFX_BOUNCE_BOUNDS k_ptBounce(DevScene s, DevFrame f, DevFrameParams p, DevPathState ps, DevRegir rg, uint32_t round,
+__global__ void __launch_bounds__(64, kBounceMinBlocks) k_ptBounce(DevScene s, DevFrame f, DevFrameParams p, DevPathState ps, DevRegir rg, uint32_t round,
                                                  uint32_t maxLengthTerminate) {
     const uint32_t curQueue = round & 1u, nextQueue = curQueue ^ 1u;
     const uint32_t* roundCounters = ps.counters + 4 * round;

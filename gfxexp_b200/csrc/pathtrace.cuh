@@ -11,6 +11,9 @@
 namespace gfx {
 
 constexpr uint32_t kMaxPathRounds = 64;
+// occupancy of the first-hit / bounce kernels: 16 blocks of 64 threads per SM = 64 registers (measured against the 88-128
+// ptxas picks unconstrained: path-tracer bounce 0.44 -> 0.37 ms, NRC bounce 0.58 -> 0.53 ms; profiles/r02_summary.md)
+constexpr int kBounceMinBlocks = 16;
 
 struct DevPathState {
     float4* alphaPdf;      // per pixel: alpha.rgb, prevDirPDensity

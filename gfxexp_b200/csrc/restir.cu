@@ -15,11 +15,13 @@
 
 namespace gfx {
 
-// PHASE 0: the whole program in one kernel, visibility traced inline (megakernel form of the reference).
+// PHASE 0: the whole program in one kernel (megakernel form of the reference), for frames without visibility reuse.
 // PHASE 1: candidates + recPDF, the visibility ray is only *requested* (wavefront form).
 // PHASE 2: applies the answered visibility, then the temporal merge.
 //
-// PHASE 1 runs the candidate loop in two phases (TWO_PHASE).  ncu on the lock-step loop (round 2, profiles/r02_summary.md):
+// PHASE 1 without an environment light runs the candidate loop in two phases (kRisTwoPhase); PHASE 0 and frames with an
+// environment light, whose candidates choose their light type by index, run it in lock step.
+// ncu on the lock-step loop (round 2, profiles/r02_summary.md):
 // ~70 % of the candidates are dark and leave after the staged light fetch, so everything after the bounding-sphere test - 74 %
 // of the kernel's issue slots - ran with 9-16 of 32 lanes.  Phase A walks all 2^n candidates in lock step but only draws ul,
 // picks the light and tests its bounding sphere (the other three draws of a candidate are skipped with the LCG's 4-step
@@ -29,9 +31,11 @@ namespace gfx {
 // lock-step loop.  A warp then iterates max-over-lanes(#survivors) ~ 20 times instead of 32, with the expensive part at
 // ~70 % instead of 30 % lane utilisation; each pixel still sees the reference's sequence of Reservoir::update calls
 // (restir_di_shared.h:118-125) and draws, so results are bit-identical.
-constexpr uint32_t kRisMaxCandidates = 32; // TWO_PHASE keeps one key per candidate and thread in shared memory
+constexpr uint32_t kRisMaxCandidates = 32; // the two-phase loop keeps one key per candidate and thread in shared memory
+template <int PHASE, bool ENV>
+constexpr bool kRisTwoPhase = PHASE == 1 && !ENV;
 
-template <bool withTemporalRIS, bool useUnbiasedEstimator, int PHASE, bool TWO_PHASE, bool ENV>
+template <bool withTemporalRIS, bool useUnbiasedEstimator, int PHASE, bool ENV>
 GFX_D bool risPixel(const DevScene &s, const DevFrame &f, const DevFrameParams &p, RayRequest* request, uint32_t* candidateKeys) {
     // optix_restir_di_kernels.cu:14-287
     const uint32_t x = blockIdx.x * 8 + threadIdx.x;
@@ -80,7 +84,7 @@ GFX_D bool risPixel(const DevScene &s, const DevFrame &f, const DevFrameParams &
     bool hasSelection = false;
     bool selEnv = false; // ENV: the selected candidate came from the environment map
     float sumWeights = 0.0f;
-    if (TWO_PHASE && numCandidates <= kRisMaxCandidates) {
+    if (kRisTwoPhase<PHASE, ENV> && numCandidates <= kRisMaxCandidates) {
         uint32_t* myKeys = candidateKeys + (threadIdx.x + threadIdx.y * blockDim.x); // [candidate][64 threads]
         const uint64_t state0 = rng.state;
         // ---- phase A: ul, light pick, bounding sphere
@@ -314,20 +318,16 @@ GFX_D bool risPixel(const DevScene &s, const DevFrame &f, const DevFrameParams &
     return false;
 }
 
-#ifndef GFX_RIS_MIN_BLOCKS
-#define GFX_RIS_MIN_BLOCKS 16 // 64 registers: measured 1.49 ms against 1.80 ms at the 84 registers ptxas picks unconstrained (profiles/r02_summary.md)
-#endif
-template <bool withTemporalRIS, bool useUnbiasedEstimator, int PHASE, bool TWO_PHASE = false, bool ENV = false>
-__global__ void __launch_bounds__(64, GFX_RIS_MIN_BLOCKS) k_initialAndTemporalRIS(DevScene s, DevFrame f, DevFrameParams p) {
-    static_assert(!TWO_PHASE || PHASE == 1, "the two-phase candidate loop belongs to the wavefront candidate pass");
-    static_assert(!(TWO_PHASE && ENV), "environment-light candidates go through the lock-step loop");
+constexpr int kRisMinBlocks = 16; // 64 registers: measured 1.49 ms against 1.80 ms at the 84 registers ptxas picks unconstrained (profiles/r02_summary.md)
+template <bool withTemporalRIS, bool useUnbiasedEstimator, int PHASE, bool ENV = false>
+__global__ void __launch_bounds__(64, kRisMinBlocks) k_initialAndTemporalRIS(DevScene s, DevFrame f, DevFrameParams p) {
     RayRequest request;
     uint32_t* candidateKeys = nullptr;
-    if constexpr (TWO_PHASE) {
+    if constexpr (kRisTwoPhase<PHASE, ENV>) {
         __shared__ uint32_t keys[kRisMaxCandidates * 64]; // [candidate][thread of the 8x8 block]
         candidateKeys = keys;
     }
-    const bool want = risPixel<withTemporalRIS, useUnbiasedEstimator, PHASE, TWO_PHASE, ENV>(s, f, p, &request, candidateKeys);
+    const bool want = risPixel<withTemporalRIS, useUnbiasedEstimator, PHASE, ENV>(s, f, p, &request, candidateKeys);
     if (PHASE == 1)
         enqueueRay(f, s.rayCounter, want, request);
 }
@@ -604,24 +604,19 @@ int launchReSTIR(gfx_ctx* ctx, cudaStream_t stream, const GfxFrameParams* params
     const dim3 grid((ctx->frame.W + 7) / 8, (p.y1 - p.y0 + 7) / 8);
     const DevScene s = ctx->devScene(params);
     const DevFrame f = ctx->devFrame();
-    // wavefront form (default): request rays -> persistent-thread trace -> resolve.  GFX_MEGAKERNEL=1 selects
-    // the single-kernel form with inline traversal (same results; kept for A/B measurements).
-    static const bool megakernel = getenv("GFX_MEGAKERNEL") != nullptr;
-    const bool wave = !megakernel;
-    // the two-phase candidate loop (see risPixel) is the default; GFX_RIS_TWO_PHASE=0 selects the lock-step loop (A/B)
-    static const bool twoPhase = !(getenv("GFX_RIS_TWO_PHASE") && getenv("GFX_RIS_TWO_PHASE")[0] == '0');
+    // with visibility reuse the RIS pass is a wavefront: request rays -> persistent-thread trace -> resolve; without it
+    // there is no ray to trace and one kernel does the pass
 #define RIS_LAUNCH(T, U) \
-    if (wave && p.reuseVisibility) { \
+    if (p.reuseVisibility) { \
         int rc_ = resetVisibilityQueue(ctx, stream); if (rc_) return rc_; \
         { GFX_TIMED(ctx, stream, "ris_candidates"); \
-          if (s.env.enabled) k_initialAndTemporalRIS<T, U, 1, false, true><<<grid, block, 0, stream>>>(s, f, p); \
-          else if (twoPhase) k_initialAndTemporalRIS<T, U, 1, true><<<grid, block, 0, stream>>>(s, f, p); \
-          else k_initialAndTemporalRIS<T, U, 1, false><<<grid, block, 0, stream>>>(s, f, p); } ctx->launches++; \
+          if (s.env.enabled) k_initialAndTemporalRIS<T, U, 1, true><<<grid, block, 0, stream>>>(s, f, p); \
+          else k_initialAndTemporalRIS<T, U, 1><<<grid, block, 0, stream>>>(s, f, p); } ctx->launches++; \
         rc_ = traceVisibilityQueue(ctx, stream); if (rc_) return rc_; \
         { GFX_TIMED(ctx, stream, "ris_resolve_temporal"); k_initialAndTemporalRIS<T, U, 2><<<grid, block, 0, stream>>>(s, f, p); } \
     } else { \
         { GFX_TIMED(ctx, stream, "ris_megakernel"); \
-          if (s.env.enabled) k_initialAndTemporalRIS<T, U, 0, false, true><<<grid, block, 0, stream>>>(s, f, p); \
+          if (s.env.enabled) k_initialAndTemporalRIS<T, U, 0, true><<<grid, block, 0, stream>>>(s, f, p); \
           else k_initialAndTemporalRIS<T, U, 0><<<grid, block, 0, stream>>>(s, f, p); } \
     }
     switch (pass) {
@@ -632,7 +627,7 @@ int launchReSTIR(gfx_ctx* ctx, cudaStream_t stream, const GfxFrameParams* params
     case GFX_RESTIR_SPATIAL_UNBIASED: { GFX_TIMED(ctx, stream, "spatial_ris_unbiased"); k_spatialRIS<true><<<grid, block, 0, stream>>>(s, f, p); } break;
     case GFX_RESTIR_SHADING: {
         const bool visDone = p.reuseVisibility && (!p.enableTemporalReuse || (p.enableSpatialReuse && p.useUnbiasedEstimator));
-        if (wave && !visDone) {
+        if (!visDone) {
             int rc_ = resetVisibilityQueue(ctx, stream); if (rc_) return rc_;
             { GFX_TIMED(ctx, stream, "shading_rays"); k_shadingRays<<<grid, block, 0, stream>>>(s, f, p); } ctx->launches++;
             rc_ = traceVisibilityQueue(ctx, stream); if (rc_) return rc_;

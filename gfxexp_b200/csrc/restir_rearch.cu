@@ -16,7 +16,6 @@
 // * shadeAndResample is a per-pixel kernel without rays.
 #include "restir_common.cuh"
 #include "wavefront.cuh"
-#include <cstdlib>
 #include <random>
 #include <vector>
 
@@ -679,12 +678,8 @@ int launchReSTIRRearch(gfx_ctx* ctx, cudaStream_t stream, const GfxFrameParams* 
         {
             GFX_TIMED(ctx, stream, "rearch_trace_shadow");
             const SampleVisibilityWriter w{ r.rayPixel, r.rayMask, r.sampleVis[p.bufferIndex] };
-            // postponed leaf tests: 1.84 -> 1.60 ms biased, 6.21 -> 5.29 ms unbiased on config 2 (GFX_TRACE_DEFER=0: immediate)
-            static const bool defer = [] { const char* e = getenv("GFX_TRACE_DEFER"); return !(e && e[0] == '0'); }();
-            if (defer)
-                k_traceWavefrontDeferred<true, false><<<wavefrontGrid(), 128, 0, stream>>>(s.bvh, r.rays, r.counters, 0u, r.counters + 1, w);
-            else
-                k_traceWavefront<true, false><<<wavefrontGrid(), 128, 0, stream>>>(s.bvh, r.rays, r.counters, 0u, r.counters + 1, w);
+            // postponed leaf tests: 1.84 -> 1.60 ms biased, 6.21 -> 5.29 ms unbiased on config 2 against immediate ones
+            k_traceWavefrontDeferred<true, false><<<wavefrontGrid(), 128, 0, stream>>>(s.bvh, r.rays, r.counters, 0u, r.counters + 1, w);
         }
         ctx->launches += 2;
     } break;

@@ -9,7 +9,6 @@
 //
 // The kernel itself (persistent threads with warp-ballot refill) lives in wavefront.cuh.
 #include "wavefront.cuh"
-#include <cstdlib>
 #include "context.h"
 
 namespace gfx {
@@ -81,12 +80,8 @@ int traceVisibilityQueue(gfx_ctx* ctx, cudaStream_t stream) {
     const FrameState &F = ctx->frame;
     VisibilityWriter w{ F.rayPixel, F.visibility };
     GFX_TIMED(ctx, stream, "trace_visibility");
-    // ReSTIR visibility rays mostly reach their light: postponed leaf tests win 10 % (GFX_TRACE_DEFER=0: immediate, A/B)
-    static const bool defer = [] { const char* e = getenv("GFX_TRACE_DEFER"); return !(e && e[0] == '0'); }();
-    if (defer)
-        k_traceWavefrontDeferred<true, false><<<wavefrontGrid(), 128, 0, stream>>>(dev.bvh, F.rayQueue, F.rayCounters, 0u, F.rayCounters + 1, w);
-    else
-        k_traceWavefront<true, false><<<wavefrontGrid(), 128, 0, stream>>>(dev.bvh, F.rayQueue, F.rayCounters, 0u, F.rayCounters + 1, w);
+    // ReSTIR visibility rays mostly reach their light: postponed leaf tests win 10 % over immediate ones
+    k_traceWavefrontDeferred<true, false><<<wavefrontGrid(), 128, 0, stream>>>(dev.bvh, F.rayQueue, F.rayCounters, 0u, F.rayCounters + 1, w);
     ctx->launches++;
     GFX_CUDA(ctx, cudaGetLastError());
     return GFX_OK;

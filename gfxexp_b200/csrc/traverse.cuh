@@ -211,33 +211,20 @@ GFX_D bool traverseStep(const DevBvh &bvh, TraversalState &st, PendingLeaves* pe
                          : 0xFFFFFFFFu;
     }
     // 19-comparator network, ascending: leaf hits (near..far), internal hits (near..far), misses.
-    // Visibility rays stop at the first hit whatever the order, so they only need leaves before internal nodes:
-    // GFX_ANYHIT_UNSORTED (A/B switch) skips the network and keeps the slot order within each group.
-#if defined(GFX_ANYHIT_UNSORTED)
-    if (!ANY_HIT) {
-#endif
     GFX_CSWAP(keys[0], keys[2]); GFX_CSWAP(keys[1], keys[3]); GFX_CSWAP(keys[4], keys[6]); GFX_CSWAP(keys[5], keys[7]);
     GFX_CSWAP(keys[0], keys[4]); GFX_CSWAP(keys[1], keys[5]); GFX_CSWAP(keys[2], keys[6]); GFX_CSWAP(keys[3], keys[7]);
     GFX_CSWAP(keys[0], keys[1]); GFX_CSWAP(keys[2], keys[3]); GFX_CSWAP(keys[4], keys[5]); GFX_CSWAP(keys[6], keys[7]);
     GFX_CSWAP(keys[2], keys[4]); GFX_CSWAP(keys[3], keys[5]);
     GFX_CSWAP(keys[1], keys[4]); GFX_CSWAP(keys[3], keys[6]);
     GFX_CSWAP(keys[1], keys[2]); GFX_CSWAP(keys[3], keys[4]); GFX_CSWAP(keys[5], keys[6]);
-#if defined(GFX_ANYHIT_UNSORTED)
-    }
-#endif
 
     // ---- leaf children: intersect their triangle chains now (shrinks best.dist before descending)
     const uint32_t leafBase = n1.y;
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
         const uint32_t key = keys[k];
-        if (key >= 0x80000000u) {
-#if defined(GFX_ANYHIT_UNSORTED)
-            if (ANY_HIT)
-                continue;
-#endif
+        if (key >= 0x80000000u)
             break;
-        }
         const uint32_t slot = key & 7u;
         const float tn = __uint_as_float((key & 0x7FFFFFF8u) << 1);
         if (tn > st.best.dist)

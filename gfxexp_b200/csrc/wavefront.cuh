@@ -10,11 +10,6 @@
 // is called exactly once per ray, by the lane that traced it.
 #pragma once
 #include "traverse.cuh"
-#include <cstdlib>
-
-#ifndef GFX_TRACE_FLUSH_LANES
-#define GFX_TRACE_FLUSH_LANES 16
-#endif
 
 namespace gfx {
 
@@ -46,7 +41,7 @@ GFX_D void traceWavefrontBody(const DevBvh &bvh, const float4* __restrict__ rays
     // immediate version: the node step runs with 27.8 of 32 lanes, the triangle tests inside it with 6-12, and they
     // issue 60 % of the warp instructions.  A lane whose traversal has ended with leaves still postponed waits
     // (`draining`) for the next flush; an occluded any-hit ray learns it at the flush.
-    constexpr int kFlushLanes = GFX_TRACE_FLUSH_LANES;
+    constexpr int kFlushLanes = 16;
     PendingLeaves pend;
     pend.n = 0;
     bool draining = false;
@@ -159,9 +154,8 @@ static inline int wavefrontGrid() {
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     // 9 x 128 threads per SM: what 56 registers admit (measured 8 / 9 / 12 / 16: 0.847 / 0.821 / 0.821 / 0.822 ms per
-    // visibility trace); GFX_TRACE_BLOCKS_PER_SM overrides (A/B)
-    static const int perSm = [] { const char* e = getenv("GFX_TRACE_BLOCKS_PER_SM"); const int v = e ? atoi(e) : 0; return v > 0 && v <= 32 ? v : 9; }();
-    return sms * perSm;
+    // visibility trace)
+    return sms * 9;
 }
 
 } // namespace gfx

@@ -169,15 +169,6 @@ class Context:
     def peer_open(self, link: int, buffer_id: int, index: int, handle: bytes):
         self._check(self.lib.gfx_peer_open(self.h, link, buffer_id, index, C.create_string_buffer(handle, 64)), "gfx_peer_open")
 
-    def peer_push_rows(self, link: int, buffer_id: int, index: int, row_lo: int, row_hi: int, stream=None):
-        self._check(self.lib.gfx_peer_push_rows(self.h, stream, link, buffer_id, index, row_lo, row_hi), "gfx_peer_push_rows")
-
-    def peer_signal(self, link: int, flag_index: int, value: int, stream=None):
-        self._check(self.lib.gfx_peer_signal(self.h, stream, link, flag_index, value), "gfx_peer_signal")
-
-    def peer_wait(self, flag_index: int, value: int, stream=None):
-        self._check(self.lib.gfx_peer_wait(self.h, stream, flag_index, value), "gfx_peer_wait")
-
     def peer_timed_out(self, stream=None) -> bool:
         v = abi.c_u32()
         self._check(self.lib.gfx_peer_status(self.h, stream, C.byref(v)), "gfx_peer_status")

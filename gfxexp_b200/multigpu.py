@@ -9,7 +9,8 @@ offsets.  Per frame:
   3. exchange of the reservoir + reservoir-info halo rows with the neighbour ranks (the spatial pass
      gathers within `spatialNeighborRadius` pixels, restir_di_main.cpp:2069; default 20).  On GPUs this is a
      one-sided push over NVLink peer memory: each rank's kernels store its seam rows into the neighbour's
-     buffers and raise a sequence flag there (csrc/peer.cu); the gloo/CPU arm uses send/recv.
+     buffers and raise a sequence flag there (csrc/peer.cu, inside gfx_restir_strip_frame); without peer links
+     (NCCL, or the gloo/CPU arm) `exchange_halo` uses send/recv.
   4. spatial RIS pass(es) on the owned rows (halo exchange again after every pass that feeds another)
   5. shading on the owned rows, exchange of the final reservoir halo (next frame's temporal reuse)
   6. all-gather of the composited beauty strips: the one mandatory collective
@@ -120,15 +121,6 @@ class GpuBackend:
 
     def restir(self, params, pass_id: int):
         self._record(abi.OP_RESTIR, pass_id, params=params)
-
-    def peer_push_rows(self, link, buffer_id, index, row_lo, row_hi):
-        self._record(abi.OP_PEER_PUSH_ROWS, link, buffer_id, index, row_lo, row_hi)
-
-    def peer_signal(self, link, flag_index, value):
-        self._record(abi.OP_PEER_SIGNAL, link, flag_index, value)
-
-    def peer_wait(self, flag_index, value):
-        self._record(abi.OP_PEER_WAIT, flag_index, value)
 
     def tensor(self, buffer_id: int, index: int = 0) -> torch.Tensor:
         key = (buffer_id, index)
@@ -243,8 +235,6 @@ class StripDriver:
         """Neighbour exchange of `halo` seam rows for the given [(buffer_id, index)] list."""
         if self.world == 1:
             return
-        if getattr(self.backend, "peer_ready", False):
-            return self._exchange_halo_peer(buffers)
         if hasattr(self.backend, "flush"):
             self.backend.flush()  # the recorded launches must be in the stream before the send/recv
         ops = []
@@ -264,26 +254,6 @@ class StripDriver:
         if ops:
             for work in dist.batch_isend_irecv(ops):
                 work.wait()
-
-    def _exchange_halo_peer(self, buffers):
-        """Push my seam rows into the neighbours' buffers, raise their flags, wait for mine (csrc/peer.cu)."""
-        b = self.backend
-        b.peer_seq += 1
-        seq = b.peer_seq
-        up, down = self.rank > 0, self.rank < self.world - 1
-        for buffer_id, index in buffers:
-            if up:
-                b.peer_push_rows(0, buffer_id, index, self.y0, min(self.y0 + self.halo, self.y1))
-            if down:
-                b.peer_push_rows(1, buffer_id, index, max(self.y1 - self.halo, self.y0), self.y1)
-        if up:
-            b.peer_signal(0, 1, seq)   # I am the upper neighbour's lower neighbour: its flag word 1
-        if down:
-            b.peer_signal(1, 0, seq)
-        if up:
-            b.peer_wait(0, seq)
-        if down:
-            b.peer_wait(1, seq)
 
     def check_peers(self):
         """raises if a seam wait timed out since the last check (a stalled neighbour: rows of this frame may be stale)"""

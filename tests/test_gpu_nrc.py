@@ -1,5 +1,5 @@
 """GPU parity: the NRC network (fused hash-grid/one-blob/identity encoding + tcgen05 MLP inference and training step;
-the CUDA-core training kernel is the A/B arm and the deep-network fallback) vs the CPU oracle.  Tensor-core accumulation order is hardware-defined, so the bar is
+the CUDA-core training kernel for networks of more than 3 hidden layers) vs the CPU oracle.  Tensor-core accumulation order is hardware-defined, so the bar is
 <= 1e-3 relative L2 on inference (BASELINE.json north_star) and agreement of loss curves / weights on training."""
 import numpy as np
 import pytest
@@ -67,22 +67,28 @@ def test_split_encoding_is_bit_exact(gfx_ctx, oracle):
     gnet.close()
 
 
-def test_fused_and_split_inference_agree(gfx_ctx, monkeypatch):
-    """GFX_NRC_INFER_FUSED=1 (hash-grid gathers from L2 inside the MLP kernel, the A/B arm) and the default split path feed the
-    same halves to the same tcgen05 MLP: identical radiance"""
+def test_fused_and_split_inference_agree(gfx_ctx):
+    """Queries or predictions that are not 16-byte aligned (here: views 4 bytes into their buffers) take the fused kernel
+    (hash-grid gathers from L2 inside the MLP kernel); aligned ones take the split path.  Both feed the same halves to the
+    same tcgen05 MLP: identical radiance"""
     import torch
     gnet = engine.NeuralRadianceCache(gfx_ctx, 2, 1e-2)
     gnet.set_params(engine.random_nrc_params(gnet.num_params, 64 * 64 * 2 + 16 * 64, seed=5, grid_amplitude=0.5))
     n = 128 * 77
     dq = torch.from_numpy(_queries(n, 2)).cuda()
-    a = torch.empty((n, 3), device="cuda")
-    b = torch.empty((n, 3), device="cuda")
-    gnet.infer(dq, a, n)
-    monkeypatch.setenv("GFX_NRC_INFER_FUSED", "1")
-    gnet.infer(dq, b, n)
-    monkeypatch.delenv("GFX_NRC_INFER_FUSED")
+    dq_offset = torch.empty(n * 14 + 1, device="cuda")[1:].view(n, 14)
+    dq_offset.copy_(dq)
+    split = torch.empty((n, 3), device="cuda")
+    fused_in = torch.empty((n, 3), device="cuda")
+    fused_out = torch.empty(n * 3 + 1, device="cuda")[1:].view(n, 3)
+    assert dq.data_ptr() % 16 == 0 and split.data_ptr() % 16 == 0 and fused_in.data_ptr() % 16 == 0
+    assert dq_offset.data_ptr() % 16 == 4 and fused_out.data_ptr() % 16 == 4
+    gnet.infer(dq, split, n)
+    gnet.infer(dq_offset, fused_in, n)
+    gnet.infer(dq, fused_out, n)
     torch.cuda.synchronize()
-    assert torch.equal(a, b)
+    assert torch.equal(split, fused_in)
+    assert torch.equal(split, fused_out)
     gnet.close()
 
 
@@ -96,12 +102,12 @@ def test_infer_rejects_unpadded_batch(gfx_ctx):
     gnet.close()
 
 
-def test_training_tracks_oracle(gfx_ctx, oracle):
+def _train_against_oracle(gfx_ctx, oracle, hidden):
     import torch
-    onet = oracle.OracleNrc(2, 1e-2)
+    onet = oracle.OracleNrc(hidden, 1e-2)
     params = engine.random_nrc_params(onet.num_params, onet.num_matrix_weights, seed=11)
     onet.set_params(params)
-    gnet = engine.NeuralRadianceCache(gfx_ctx, 2, 1e-2)
+    gnet = engine.NeuralRadianceCache(gfx_ctx, hidden, 1e-2)
     gnet.set_params(params)
     n = 4096
     q = _queries(n, 9)
@@ -123,35 +129,15 @@ def test_training_tracks_oracle(gfx_ctx, oracle):
     gnet.close()
 
 
-def test_tensor_core_training_matches_cuda_core_training(gfx_ctx):
-    """The tcgen05 training kernel (forward, data and weight gradients as MMAs) and the CUDA-core kernel implement the
-    same step with the same fp16 rounding points; only the fp32 accumulation order differs."""
-    import os
-    import torch
-    n = 8192
-    q = _queries(n, 21)
-    target = np.stack([0.5 + 0.4 * np.sin(6 * q[:, 0]), q[:, 1] * q[:, 8], 0.3 + 0.5 * q[:, 2]], axis=1).astype(np.float32)
-    dq, dt = torch.from_numpy(q).cuda(), torch.from_numpy(target).cuda()
-    results = {}
-    for arm in ("0", "1"):
-        os.environ["GFX_NRC_TRAIN_CUDACORES"] = arm
-        try:
-            net = engine.NeuralRadianceCache(gfx_ctx, 2, 1e-2)
-            net.set_params(engine.random_nrc_params(net.num_params, 64 * 64 * 2 + 16 * 64, seed=3))
-            losses = [net.train(dq, dt, n, want_loss=True) for _ in range(10)]
-            out = torch.empty((n, 3), dtype=torch.float32, device="cuda")
-            net.infer(dq, out, n)
-            torch.cuda.synchronize()
-            results[arm] = (np.array(losses), out.cpu().numpy())
-            net.close()
-        finally:
-            os.environ.pop("GFX_NRC_TRAIN_CUDACORES", None)
-    (l0, o0), (l1, o1) = results["0"], results["1"]
-    assert np.isfinite(l0).all() and np.isfinite(o0).all()
-    assert abs(l0[0] - l1[0]) <= 1e-5 * abs(l1[0])        # same forward pass on the same weights
-    assert np.abs(l0 - l1).max() <= 0.03 * l1.max(), (l0, l1)
-    assert l0[-1] < 0.5 * l0[0]
-    assert _rel_l2(o0, o1) <= 2e-2, _rel_l2(o0, o1)
+def test_training_tracks_oracle(gfx_ctx, oracle):
+    """2 hidden layers: the tcgen05 training kernel (forward, data and weight gradients as MMAs)"""
+    _train_against_oracle(gfx_ctx, oracle, 2)
+
+
+def test_cuda_core_training_tracks_oracle(gfx_ctx, oracle):
+    """4 hidden layers, the shallowest network whose activation tiles do not fit the tcgen05 training kernel's shared
+    memory: the CUDA-core training kernel"""
+    _train_against_oracle(gfx_ctx, oracle, 4)
 
 
 def test_tensor_core_training_is_deterministic(gfx_ctx):

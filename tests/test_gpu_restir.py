@@ -48,21 +48,29 @@ def test_light_distributions(gfx_ctx, oracle):
     assert integ > 0
 
 
-@pytest.mark.parametrize("unbiased,scene_name", [(False, "small_city_scene"), (True, "small_city_scene"),
-                                                 (False, "small_interior_scene"),
-                                                 # environment light: importance-map candidates, atInfinity samples through
-                                                 # temporal / spatial reuse, the environment behind miss pixels
-                                                 (False, "small_city_scene_env"), (True, "small_city_scene_env"),
-                                                 (False, "env_only_scene"),
-                                                 # image textures on the BSDF parameters (software tex2DLod, repeat addressing)
-                                                 (False, "small_city_scene_textured")])
-def test_restir_three_frames_bit_exact(gfx_ctx, oracle, unbiased, scene_name):
+_THREE_FRAME_CASES = [(False, "small_city_scene", 1), (True, "small_city_scene", 1),
+                      (False, "small_interior_scene", 1),
+                      # environment light: importance-map candidates, atInfinity samples through
+                      # temporal / spatial reuse, the environment behind miss pixels
+                      (False, "small_city_scene_env", 1), (True, "small_city_scene_env", 1),
+                      (False, "env_only_scene", 1),
+                      # image textures on the BSDF parameters (software tex2DLod, repeat addressing)
+                      (False, "small_city_scene_textured", 1),
+                      # no visibility reuse: the RIS pass is one kernel without a ray queue (with and without the
+                      # environment light), the spatial passes evaluate unshadowed target densities
+                      (False, "small_city_scene", 0), (True, "small_city_scene", 0), (False, "small_city_scene_env", 0)]
+
+
+@pytest.mark.parametrize("unbiased,scene_name,reuse_visibility", _THREE_FRAME_CASES,
+                         ids=[f"{u}-{s}" + ("" if v else "-no_reuse_visibility") for u, s, v in _THREE_FRAME_CASES])
+def test_restir_three_frames_bit_exact(gfx_ctx, oracle, unbiased, scene_name, reuse_visibility):
     # small_interior_scene: config 3's ingredients - a closed room, 96 two-triangle emitters, SimplePBR materials
     # (common/common_device.cuh:767-776, 806-826)
     scene = getattr(scenes, scene_name)()
     w, h = 192, 108
     oscene, oframe = _setup(gfx_ctx, oracle, scene, w, h)
     p = abi.default_frame_params(scene, w, h)
+    p.reuseVisibility = reuse_visibility
     for frame in range(3):
         gfx_ctx.build_light_distributions(frame % 2)
         for kind, pass_id in engine.restir_frame_passes(p, frame, num_spatial_passes=2 if not unbiased else 1,
